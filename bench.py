@@ -2,6 +2,7 @@
 """bench.py -- the driver-facing benchmark of the fused ABFT-SGEMM hot path.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size n] [--id KERNEL_ID] [--sweep]
+                  [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input: one fused fault-tolerant SGEMM
 C = alpha*A*B^T + beta*C (encode pre-pass + tcgen05 kernel with checksum tile-columns, per-tile detect/correct) at
@@ -16,6 +17,12 @@ The JSON line also carries: `sweep` (N=1: fused ABFT / own plain kernel / cuBLAS
 number of launches per cell, engines interleaved), `strong` (BASELINE.json configs[4]: ONE 32768^3 product on the P x Q
 rank grid, incl. the verdict exchange), `id16` (configs[1] literally: the 128x128x8 tile), `parity` (sampled rows of the
 bench's own result against the CPU oracle, outside the timed regions).
+
+--dump-outputs DIR writes C as the last timed step left it, so that two builds can be compared output for output: the inputs
+are seeded, so the same arguments give the same inputs on every run.  DIR/C_rows.npy (float32) holds rows of the M x N
+result, DIR/C_row_index.npy (float64) which rows: all of them when they fit the budget, else a fixed seeded sample.  All
+files together stay within DUMP_BYTES: under torchrun every rank writes C_rows_rank<r>.npy / C_row_index_rank<r>.npy for
+its own C block within DUMP_BYTES / world.  (--impl reference has no GPU output to dump and refuses the option.)
 
 --impl reference times the reference's own CPU SGEMM (cpu_gemm, utils/utils.cu:79-89, compiled unmodified into
 oracle/_ref/libref_utils.so; falls back to the OpenMP oracle port) on the host cores; rank 0 only.
@@ -37,6 +44,7 @@ sys.path.insert(0, str(ROOT))
 
 METRIC = "fused ABFT SGEMM GFLOPS (2*M*N*K/t) and ABFT overhead % vs cuBLAS-TF32, M=N=K=4096"
 README_ABFT_HUGE_4096 = 4005.0  # BASELINE.md section 1 (README.md:53), hardware unspecified
+DUMP_BYTES = 32 << 20  # --dump-outputs: at most this much in all ranks' files together (half of C at the default 4096^2)
 
 
 def _peaks():
@@ -242,6 +250,19 @@ def fill_ref_dist(t, gen):
     return t
 
 
+def sample_rows(dC, M, N, budget):
+    """Rows of C (column-major M x N on the device) for --dump-outputs: (row index as float64, those rows as float32),
+    together at most `budget` bytes."""
+    import numpy as np
+    import torch
+    R = min(M, budget // (4 * N + 8))
+    if R < 1:
+        raise ValueError(f"--dump-outputs: one row of C ({4 * N} bytes) exceeds the budget of {budget} bytes")
+    rows = np.arange(M) if R == M else np.sort(np.random.default_rng(0).choice(M, R, replace=False))
+    got = dC.view(N, M).t()[torch.from_numpy(rows).to(dC.device)].cpu().numpy()
+    return rows.astype(np.float64), got
+
+
 def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
@@ -260,7 +281,12 @@ def main():
     ap.add_argument("--id", type=int, default=31, help="fused ABFT kernel id (31 = 256x256 CTA-pair tile, 16 = literal huge 128x128)")
     ap.add_argument("--no-sweep", action="store_true", help="skip the 1024..16384 sweep (N=1)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write C of the last timed step to DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs dumps the GPU path's C; --impl reference has none")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -284,7 +310,7 @@ def main():
     P, Q = sharding.shard_grid(world)
     alpha, beta = 1.0, -1.5
     W = max(args.warmup, 3)
-    steps = max(1, args.steps)
+    steps = args.steps
     g = torch.Generator(device="cuda").manual_seed(1234 + rank)
     ft = pkg.FtSgemm()
     stream = torch.cuda.current_stream().cuda_stream
@@ -396,6 +422,7 @@ def main():
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     verdict = exch.verdict() if exch is not None else (peer.verdict() if peer is not None else None)
     st = ft.stats()
+    dump = sample_rows(prob.dC, M, N, DUMP_BYTES // world) if args.dump_outputs else None  # (the comparators below overwrite C)
     ms_step = ms_total / steps
     value = world * flops_per_step / (ms_step * 1e-3) / 1e9
     comp["plain"] = prob.time_engine(plain_id, steps)
@@ -543,6 +570,13 @@ def main():
                            " + verdict exchange (NCCL all-gather of the device-side vectors)") if world > 1 else "")}
             del sp
             torch.cuda.empty_cache()
+
+    if dump is not None:
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        sfx = f"_rank{rank}" if world > 1 else ""
+        np.save(out_dir / f"C_row_index{sfx}.npy", dump[0])
+        np.save(out_dir / f"C_rows{sfx}.npy", dump[1])
 
     if rank != 0:
         if dist is not None:
