@@ -616,6 +616,12 @@ int run_tc(ftsgemm_handle_t h, const Variant &v, int M, int N, int K, const floa
     p.chk_slices = p.chk_in_carriers ? 1 : choose_chk_slices(p, max_units, K);
     const size_t n_flags_s = static_cast<size_t>(p.tiles_m) * CG * (kBM / 32) * p.tiles_c * p.chk_slices;
     if (p.chk_slices > 1 && n_flags_s * sizeof(int) > kChkFlagBytes) p.chk_slices = 1;
+    // Default tau_rel beyond K = 8192 (DESIGN.md section 5): with non-negative operands the accumulator's truncation-like
+    // rounding adds up with K instead of cancelling, so the fault-free residual grows like K: 1e-5 * K / 8192.  Checksum
+    // K-slices restart the expected checksum's accumulation and the data row's rounding no longer cancels against it:
+    // 2.5e-8 * K (measured U[0,1) operands, (1024, 1024, K): 5.2e-9 * K; K = 16384 .. 65536 were all flagged at 1e-5).
+    if (!(o.tau_rel > 0))
+      p.tau_rel = fmaxf(1e-5f, (p.chk_slices > 1 ? 2.5e-8f : 1e-5f / 8192.0f) * static_cast<float>(K));
     if (p.chk_slices > 1) {
       // one plane of expected checksums per slice
       const size_t out_floats = static_cast<size_t>(M) * p.n_chk_cols * p.chk_slices;

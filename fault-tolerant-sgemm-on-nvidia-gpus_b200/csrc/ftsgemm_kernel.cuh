@@ -510,13 +510,17 @@ __device__ __forceinline__ void abft_check(const KernelParams &p, uint32_t taddr
   const float r1 = xp.e0 + xp.e1, r2 = xp.w0 + xp.w1;
   const float d1 = r1 - s1, d2 = r2 - s2;
   const float thr = p.tau_abs + p.tau_rel * sabs;
-  const bool flagged = !(fabsf(d1) <= thr);  // also true for NaN
+  // Expected checksum AND row sum non-finite: Inf / NaN in the operands (this row of A, or a column of B in this tile), a
+  // legitimately non-finite product that no checksum can verify.  Stored as computed, not flagged: recomputing it would only
+  // re-round its finite elements (DESIGN.md section 3.3).  An upset makes one of the two non-finite, never both.
+  const bool unverifiable = !isfinite(r1) && !isfinite(s1);
+  const bool flagged = !unverifiable && !(fabsf(d1) <= thr);  // also true for NaN
   const unsigned flag_mask = __ballot_sync(0xffffffffu, flagged);
 
   // fault-free residual statistics (threshold calibration, DESIGN.md section 5)
   {
-    float ra = flagged ? 0.0f : fabsf(d1);
-    float rr = flagged ? 0.0f : fabsf(d1) / fmaxf(sabs, 1e-30f);
+    float ra = (flagged || unverifiable) ? 0.0f : fabsf(d1);
+    float rr = (flagged || unverifiable) ? 0.0f : fabsf(d1) / fmaxf(sabs, 1e-30f);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       ra = fmaxf(ra, __shfl_xor_sync(0xffffffffu, ra, o));

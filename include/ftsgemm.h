@@ -103,7 +103,9 @@ typedef struct ftsgemm_opts {
   int n_faults;
   ftsgemm_fault faults[FTSGEMM_MAX_FAULTS];
   /* detection threshold: a row is flagged when |expected - actual row checksum| > tau_abs + tau_rel * sum_n|acc|.
-   * <= 0 selects the calibrated defaults (DESIGN.md section 5).  The reference uses the constant 9500
+   * <= 0 selects the calibrated defaults (DESIGN.md section 5): tau_abs = 1e-3, tau_rel = max(1e-5, 1.2e-9 * K), or
+   * max(1e-5, 2.5e-8 * K) when the checksum items run as K-slices -- measured fault-free floors of |d1| / sum|acc|: <= 2.3e-6
+   * up to 16384^3 on zero-mean operands, ~5.2e-9 * K with non-negative operands and K-slices.  The reference uses the constant 9500
    * (ft_sgemm_huge.cuh:50). */
   float tau_abs, tau_rel;
   int detect_only;       /* 1: count detections but do not correct */
